@@ -152,7 +152,8 @@ class ClockSampler:
 # ---- CPU arm: the oracle port of the reference path -------------------------------------------------------
 def cpu_reference_arm(steps, warmup, budget_s=20.0):
     """_loss + backward + Adam of the reference network (oracle restatement, torch CPU fp32, all host threads)
-    on GUM minibatches of 256 traces (four pre-generated minibatches cycled, like the GPU arm).  Returns traces/s."""
+    on GUM minibatches of 256 traces (four pre-generated minibatches cycled, like the GPU arm).  Returns traces/s.
+    Times `steps` steps, or fewer once `budget_s` seconds are spent (budget_s=None: exactly `steps`)."""
     from oracle import network as onet
     from oracle import params as oparams
     from pyprob_b200 import synthetic
@@ -202,13 +203,21 @@ def cpu_reference_arm(steps, warmup, budget_s=20.0):
     for _ in range(steps):
         one_step()
         done += 1
-        if time.perf_counter() - t0 > budget_s:
+        if budget_s is not None and time.perf_counter() - t0 > budget_s:
             break
     dt = time.perf_counter() - t0
     return {'value': done * BATCH / dt, 'unit': 'traces/s', 'cores': threads, 'kind': 'port',
             'sample': '{} steps of _loss+backward+Adam on {}-trace GUM minibatches (oracle/network.py, torch CPU fp32, '
                       '{} of {} host threads — the fastest setting for this small-GEMM step), {:.1f} s'.format(
                           done, BATCH, threads, os.cpu_count(), dt)}, dt / done
+
+
+def dump_outputs(out_dir, tensors):
+    """Write each tensor as out_dir/<name>.npy, float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+    log('outputs of the last timed step written to {}'.format(out_dir))
 
 
 def log(msg):
@@ -234,7 +243,16 @@ def main():
     ap.add_argument('--cpu-budget', type=float, default=15.0, help='seconds of CPU work for the cpu_baseline sample')
     ap.add_argument('--nccl-allreduce', action='store_true',
                     help='N>1: NCCL all-reduce + local Adam instead of the fused peer-memory optimiser step')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (loss, updated parameters, gradient, '
+                         'Adam moments; rank 0) as DIR/<name>.npy in float32, to compare two builds output for output. '
+                         'The inputs are seeded; the backward pass accumulates with atomics, so two runs agree to float '
+                         'rounding, not bit for bit')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 arm')
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -243,7 +261,7 @@ def main():
     if args.impl == 'reference':
         if rank != 0:
             return
-        cb, s_per_step = cpu_reference_arm(args.steps, warmup, budget_s=120.0)
+        cb, s_per_step = cpu_reference_arm(args.steps, warmup, budget_s=None)
         print(json.dumps({'impl': 'reference', 'metric': 'ic_train_traces_per_sec', 'value': cb['value'],
                           'unit': 'traces/s', 'n_gpus': args.gpus, 'steps': args.steps, 'warmup': warmup,
                           'ms_per_step': s_per_step * 1e3, 'higher_is_better': True, 'scaling': 'weak',
@@ -373,6 +391,10 @@ def main():
         run_step(i)
         ev[i][1].record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:
+        # taken before the launch count below runs one more step on the same parameters
+        dump_outputs(args.dump_outputs, {'loss': loss, 'parameters': net._arena.data, 'gradient': grad,
+                                         'adam_exp_avg': net._exp_avg, 'adam_exp_avg_sq': net._exp_avg_sq})
     # graph replays bypass the library's host-side launch counter: count the launches of one eager step
     l0 = _lib.call('ppb_launch_count')
     device_step(0)

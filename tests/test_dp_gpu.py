@@ -31,9 +31,9 @@ def _reference_steps(p, grads, world, dev):
     return p, m, v
 
 
-def test_peer_adam_single_rank_is_plain_adam():
+def test_peer_adam_single_rank_is_plain_adam(cuda):
     from pyprob_b200 import parallel
-    dev = torch.device('cuda', 0)
+    dev = cuda
     gen = torch.Generator(device='cpu').manual_seed(5)
     p0 = torch.randn(N, generator=gen).to(dev)
     grads = [torch.randn(N, generator=gen).to(dev) for _ in range(STEPS)]

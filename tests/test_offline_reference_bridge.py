@@ -1,74 +1,56 @@
-"""Build container only (skipped where /root/reference is absent, e.g. on the GPU box): real reference Trace objects
--> TraceColumns.from_reference_traces -> trace file -> OfflineDataset.batch must describe the same minibatch as the
-reference's own Batch: the oracle loss on the re-read arrays equals the UNMODIFIED reference's _loss on the traces."""
-import contextlib
-import io
+"""Reference Trace objects -> TraceColumns.from_reference_traces -> trace file -> OfflineDataset.batch must describe the
+same minibatch as the reference's own Batch: the oracle loss on the re-read arrays equals the UNMODIFIED reference's
+_loss on the traces.  The traces, the reference Batch's grouping, the network and the loss are stored golden data
+(tests/golden/make_bridge_golden.py); the traces are rebuilt here as objects with the attributes the bridge reads."""
+import json
 import os
-import sys
+from types import SimpleNamespace
 
 import numpy as np
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isdir('/root/reference/pyprob'), reason='needs the reference checkout')
+
+
+def _golden():
+    z = np.load(os.path.join(ROOT, 'tests', 'golden', 'bridge_golden.npz'))
+    params = {k[len('param.'):]: torch.from_numpy(z[k]) for k in z.files if k.startswith('param.')}
+    return json.loads(str(z['meta'])), params
+
+
+def _distribution(name, num_categories, prior):
+    fields = {'Normal': ('mean', 'stddev'), 'Uniform': ('low', 'high')}.get(name, ())
+    attrs = dict(zip(fields, prior))
+    if name == 'Categorical':
+        attrs['num_categories'] = num_categories
+    return type(name, (), attrs)()
+
+
+def _trace(rec):
+    ctrl = [SimpleNamespace(address=v['address'], value=torch.tensor(v['value']),
+                            distribution=_distribution(v['distribution'], v['num_categories'], v['prior']))
+            for v in rec['controlled']]
+    named = {nm: SimpleNamespace(value=torch.tensor(val)) for nm, val in rec['observed'].items()}
+    return SimpleNamespace(variables_controlled=ctrl, named_variables=named)
 
 
 def test_reference_traces_survive_the_columnar_store(tmp_path):
-    sys.path.insert(0, os.path.join(ROOT, 'oracle', 'ref_stubs'))
-    sys.path.insert(1, '/root/reference')
-    try:
-        import pyprob
-        from pyprob import InferenceNetwork, Model
-        from pyprob.distributions import Categorical, Normal, Poisson, Uniform
-        from pyprob.nn.dataset import Batch, OnlineDataset
-    finally:
-        sys.path.remove('/root/reference')
-        sys.path.remove(os.path.join(ROOT, 'oracle', 'ref_stubs'))
     from oracle import network as onet
     from pyprob_b200 import offline
 
-    class Branching(Model):
-        def forward(self):
-            u = pyprob.sample(Uniform(-1, 2))
-            k = pyprob.sample(Categorical([0.2, 0.3, 0.5]))
-            if int(k) == 0:
-                z = pyprob.sample(Normal(u, 0.5))
-            else:
-                z = pyprob.sample(Poisson(3.0)) * 0.25
-            mu = pyprob.sample(Normal(z * 0.1, 1))
-            pyprob.observe(Normal(mu, 0.3), name='y0')
-            pyprob.observe(Normal(u, 0.7), name='y1')
-            return mu
-
-    pyprob.set_verbosity(0)
-    pyprob.seed(5)
-    model = Branching()
-    emb = {'y0': {'dim': 8, 'depth': 2}, 'y1': {'dim': 4, 'depth': 1}}
-    with contextlib.redirect_stdout(io.StringIO()):
-        model.learn_inference_network(num_traces=48, batch_size=24, inference_network=InferenceNetwork.LSTM,
-                                      observe_embeddings=emb, lstm_dim=16, proposal_mixture_components=3)
-    net = model._inference_network
-    ds = OnlineDataset(model)
-    traces = [ds[i] for i in range(40)]
-    batch = Batch(traces)
-    with contextlib.redirect_stdout(io.StringIO()):
-        net._polymorph(batch)
-    with torch.no_grad():
-        ok, ref_loss = net._loss(batch)
-    assert ok
-    names = list(emb.keys())
+    meta, params = _golden()
+    traces = [_trace(rec) for rec in meta['traces']]
+    names = list(meta['observe_embeddings'])
     cols = offline.TraceColumns.from_reference_traces(traces, names)
     offline.save_columns(str(tmp_path), cols)
     data = offline.OfflineDataset(str(tmp_path))
-    assert len(data) == 40 and data.num_trace_types == len(batch.sub_batches)
+    assert len(data) == 40 and data.num_trace_types == len(meta['sub_batch_sizes'])
     arr = data.batch(list(range(40)))
     # same grouping as the reference Batch: sub-batches in order of first appearance, same sizes
-    assert [sb['values'].shape[1] for sb in arr.subs] == [len(sb) for sb in batch.sub_batches]
-    assert [sb['addresses'] for sb in arr.subs] == [[v.address for v in sb[0].variables_controlled]
-                                                     for sb in batch.sub_batches]
-    params = {k: v.detach() for k, v in net.state_dict().items()}
+    assert [sb['values'].shape[1] for sb in arr.subs] == meta['sub_batch_sizes']
+    assert [sb['addresses'] for sb in arr.subs] == meta['sub_batch_addresses']
     tsubs = [{k: (torch.from_numpy(np.ascontiguousarray(v)) if isinstance(v, np.ndarray) else v) for k, v in sb.items()}
              for sb in arr.subs]
-    got, _ = onet.loss(params, tsubs, names, [1, 1], 3)
-    assert abs(float(got) - float(ref_loss)) <= 2e-6 * abs(float(ref_loss))
+    got, _ = onet.loss(params, tsubs, names, [1, 1], meta['mixture_components'])
+    ref_loss = meta['loss']
+    assert abs(float(got) - ref_loss) <= 2e-6 * abs(ref_loss)
